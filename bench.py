@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA, sm_100a)
   python bench.py --impl reference --gpus N ...            reference arm: the reference's CPU path
                                                            (restated, oracle/cpu_engine.cpp) on host cores
+  python bench.py ... --dump-outputs DIR                   also write what the last timed step received (.npy)
 Every line also carries `sweep`: BASELINE config 3 sampled at 64 B ... 1 GiB in the same run (--no-sweep skips it;
 the full 25-size sweep, uni- and bidirectional, is `bench_scenarios.py sweep`).
 
@@ -186,6 +187,29 @@ async def window_step(server, client, eps, srcs, dsts):
     return [await f for f in recvs]
 
 
+DUMP_SAMPLE = 1 << 22  # received bytes kept by --dump-outputs: 16 MiB as float32, far below the 64 MB the dump may take
+
+
+def dump_outputs(out_dir, torch, dsts, results):
+    """Writes what the receiver got in one step, as a caller of window_step sees it:
+      recv_results.npy  float64 (window, 2): (sender_tag, length) of every receive, in posting order
+      recv_bytes.npy    float32: the received bytes, the window's buffers end to end; above DUMP_SAMPLE bytes a
+                        sample at sorted positions drawn from a fixed seed (the same positions for the same arguments)
+    The sample is gathered buffer by buffer, so no copy of the whole window is made."""
+    import numpy as np
+
+    total = sum(d.numel() for d in dsts)
+    pos = np.arange(total) if total <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).integers(0, total, DUMP_SAMPLE))
+    parts, start = [], 0
+    for d in dsts:
+        lo, hi = np.searchsorted(pos, [start, start + d.numel()])
+        parts.append(d[torch.from_numpy(pos[lo:hi] - start).to(d.device)].cpu())
+        start += d.numel()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "recv_results.npy"), np.asarray(results, dtype=np.float64))
+    np.save(os.path.join(out_dir, "recv_bytes.npy"), torch.cat(parts).numpy().astype(np.float32))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -245,11 +269,13 @@ def run_ours(args):
         torch.cuda.synchronize()
 
         async def timed(nsteps, srcs, dsts, sync):
+            res = None
             for i in range(nsteps):
                 k = i % POOL_SETS
                 res = await window_step(server, client, eps, srcs[k], dsts[k])
                 assert all(r == (TAG, msg) for r in res)
             sync()
+            return res
 
         # the set-up garbage (torch import, buffer lists) goes to the permanent generation: full
         # collections inside the timed region would otherwise walk ~10^6 objects (same in the reference arm)
@@ -280,6 +306,11 @@ def run_ours(args):
             bad = int(t[0])
         assert bad == 0, f"payload mismatch: {bad} of {world * window} messages differ from the sender's sources"
         payload_check = (f"asserted on every rank: {world} x {window} messages bit-exact vs the sending rank's regenerated sources")
+        if args.dump_outputs:
+            # the set the last timed step fills may have been filled by the warm-up already: clear it, so that what
+            # --dump-outputs writes can only have come from the timed steps
+            for d in dst[(args.steps - 1) % POOL_SETS]:
+                d.fill_(0xEE)
         barrier()
         torch.cuda.synchronize()
         warm_batches = ctx.stats()["pull_batches"]
@@ -289,7 +320,7 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         t0 = time.perf_counter()
-        await timed(args.steps, src, dst, torch.cuda.synchronize)
+        last_res = await timed(args.steps, src, dst, torch.cuda.synchronize)
         t1 = time.perf_counter()
         e1.record()
         e1.synchronize()
@@ -309,6 +340,8 @@ def run_ours(args):
         st["_per_rank"] = per_rank
         step_bytes = window * msg
         value = world * step_bytes * args.steps / (ms * 1e-3) / 1e9
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, torch, dst[(args.steps - 1) % POOL_SETS], last_res)
 
         # ---- the metric's "vs size" half: sampled sweep (config 3) at this N, same run
         def allreduce_max(x):
@@ -529,7 +562,7 @@ def cpu_baseline_run(msg, window, budget_s=12.0, steps=None, warmup=2):
             await step()
             n += 1
             el = time.perf_counter() - t0
-            if (steps is not None and n >= steps) or (steps is None and el > budget_s) or el > 150:
+            if (steps is not None and n >= steps) or (steps is None and el > budget_s):
                 break
         await c.aclose()
         await s.aclose()
@@ -624,7 +657,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer e2e leg (ncu launch lists of the device-resident steps)")
     ap.add_argument("--no-sweep", action="store_true", help="skip the sampled size sweep (config 3)")
     ap.add_argument("--sweep-max-bytes", type=int, default=1 << 30)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what rank 0 received in the last one as DIR/<name>.npy (CUDA arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs is written by the CUDA arm only; run it without --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
